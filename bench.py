@@ -2,6 +2,7 @@
 """bench.py -- throughput of the batched 1-D complex FFT hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4|c1] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  The default workload is
 BASELINE.json configs[1]: batched N=2^20 complex-f32 forward FFT, batch 4096, on one B200.  With
@@ -14,6 +15,9 @@ region; `roofline` relates the dominant kernel's algorithmic bytes (16 B/sample 
 f64: read once + write once, SURVEY.md 8d) to the measured HBM peak; `cpu_baseline` is the oracle
 (C restatement of the reference CPU algorithm; the Rust reference cannot be built in this image)
 timed on the host cores on a bounded sample.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's share) to DIR as .npy files, so that two
+builds can be compared output for output: the inputs are the same hash-generated data in every run.
 """
 import argparse
 import json
@@ -161,8 +165,12 @@ def run_reference(args, n, batch, real, rank, world):
         O.transform_batch(x, O.FFT, threads, timing=True)
     total = 0.0
     for _ in range(args.steps):
-        _, s = O.transform_batch(x, O.FFT, threads, timing=True)
+        y, s = O.transform_batch(x, O.FFT, threads, timing=True)
         total += s
+    dumped = None
+    if args.dump_outputs:
+        import torch
+        dumped = dump_outputs(args.dump_outputs, torch.from_numpy(y))
     value = sample * n * args.steps / total
     base = {"value": value, "unit": "complex samples/s", "cores": threads, "kind": "port", "build": O.timing_build(),
             "sample": f"{sample} transforms of N={n} per step ({per_thread} per thread)"}
@@ -176,6 +184,7 @@ def run_reference(args, n, batch, real, rank, world):
                 "sample of the workload per step",
         "cpu_baseline": base,
         "e2e": {"value": value, "unit": "complex samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
+        **({"dump": dumped} if dumped else {}),
     }))
 
 
@@ -210,7 +219,26 @@ def numa_bind(local_rank):
         return prev, f"not bound ({type(e).__name__})"
 
 
-def run_distributed(args, rank, local_rank, world, barrier, log2n=None, steps=None):
+DUMP_BYTES = 48 << 20   # sample budget of --dump-outputs: with the .npy headers the files stay below 64 MB in all
+
+
+def dump_outputs(out_dir, rows):
+    """Writes the complex tensor `rows` ([count, length], device or host) to out_dir: output.npy, float32 or float64
+    [k, length, 2] (real, imaginary), and output_rows.npy, float64 [k], the index of each row written.  All rows
+    when they fit DUMP_BYTES, else k rows drawn with a fixed seed, in ascending order.  Returns the JSON record."""
+    import torch
+    count, length = rows.shape
+    k = max(1, min(count, DUMP_BYTES // (length * rows.element_size())))
+    idx = np.arange(count) if k == count else np.sort(np.random.default_rng(0).choice(count, k, replace=False))
+    sample = torch.view_as_real(rows[torch.from_numpy(idx).to(rows.device)]).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output.npy"), sample)
+    np.save(os.path.join(out_dir, "output_rows.npy"), idx.astype(np.float64))
+    return {"dir": out_dir, "files": ["output.npy", "output_rows.npy"], "rows": k, "of_rows": count,
+            "row_length": length, "dtype": str(sample.dtype)}
+
+
+def run_distributed(args, rank, local_rank, world, barrier, log2n=None, steps=None, dump_dir=None):
     """BASELINE configs[4]: ONE transform of N = 2^30 (or 2^--log2n) samples block-distributed over the ranks.
     Returns the record (rank 0) or None."""
     import torch
@@ -244,6 +272,8 @@ def run_distributed(args, rank, local_rank, world, barrier, log2n=None, steps=No
             cur, oth = (out, oth if out is cur else cur)
         stop.record()
         barrier()
+    # rank 0's block of the last step's result, in rows of n2 samples
+    dumped = dump_outputs(dump_dir, cur.view(-1, n2)) if dump_dir and rank == 0 else None
     ms = torch.tensor([start.elapsed_time(stop)], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -293,6 +323,7 @@ def run_distributed(args, rank, local_rank, world, barrier, log2n=None, steps=No
                      "traffic": None, "peak_source": peak_src,
                      "note": f"local sweeps only: {sweeps} read+write sweeps of the rank's block per step"},
         "gpu_launches": launches_per_step * steps, "clocks": clocks.summary(),
+        **({"dump": dumped} if dumped else {}),
     }
 
 
@@ -483,7 +514,12 @@ def main():
     ap.add_argument("--exchange", default="fused", choices=["fused", "peer", "nccl"],
                     help="c5 only: exchanges folded into the row FFTs' stores over NVLink peer memory, as one kernel "
                          "each over peer memory, or pack + NCCL all_to_all + unpack")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output (rank 0; a fixed, seeded sample of its rows when larger "
+                         "than 48 MB) to DIR/output.npy, the indices of those rows to DIR/output_rows.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -516,7 +552,7 @@ def main():
         torch.cuda.synchronize()
 
     if args.workload == "c5":
-        rec = run_distributed(args, rank, local_rank, world, barrier)
+        rec = run_distributed(args, rank, local_rank, world, barrier, dump_dir=args.dump_outputs)
         if rank == 0:
             print(json.dumps(rec))
         if world > 1:
@@ -527,6 +563,8 @@ def main():
         batch = max(1, batch // world)   # BASELINE configs[2]: the batch of 65536 is sharded over the GPUs
     out, plan, x, y = run_batched(args, args.workload, batch, rank, local_rank, world, barrier, args.steps,
                                   "strong" if args.workload == "c3" else "weak", keep_output=True)
+    if args.dump_outputs and rank == 0:
+        out["dump"] = dump_outputs(args.dump_outputs, y)
     e2e = None if args.no_e2e else run_e2e(args, plan, x, y, n, real, batch, rank, local_rank, world, barrier)
     plan.close()
     del x, y

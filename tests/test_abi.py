@@ -1,6 +1,7 @@
 """CPU-side checks of the drop-in boundary: the C-ABI library loads, exports every symbol that
 include/fourier.h and include/fourier_b200.h declare, the drop-in programs compile and link against
 it, and the host-side mirror of the reference interface behaves.  No compute calls (no GPU here)."""
+import json
 import os
 import re
 import shutil
@@ -69,20 +70,31 @@ def test_dropin_programs_compile_and_link(tmp_path, libfourier, src, cc, flags):
     assert exe.exists()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/fourier-ffi"), reason="reference checkout not present")
 @pytest.mark.parametrize("src,cc,hdr", [
     ("test.c", "gcc", "ours"), ("test.cpp", "g++", "ours"), ("test.c", "gcc", "reference"),
     ("test.cpp", "g++", "reference")])
 def test_reference_ffi_tests_link_unmodified(tmp_path, libfourier, src, cc, hdr):
     """The reference's own FFI test programs (fourier-ffi/test.c, test.cpp), compiled with the
     reference's warning flags (CMakeLists.txt:9-13) against either header, link against libfourier.so
-    with no undefined symbols.  (They are run on the GPU box by tests/test_gpu_parity.py through the
-    equivalent programs in tests/ffi/, because /root/reference does not exist there.)"""
-    inc = INCLUDE if hdr == "ours" else "/root/reference/fourier-ffi/include"
+    with no undefined symbols.  tests/golden/reference_ffi_symbols.json holds the library symbols each
+    compiled program references; a program of the same language that references exactly those symbols
+    is linked here, and the symbols compiled against our header must be ones include/fourier.h declares.
+    (The equivalent programs in tests/ffi/ are run by tests/test_gpu_parity.py.)"""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_ffi_symbols.json")) as f:
+        symbols = json.load(f)["programs"][src][hdr]
+    assert set(_lib.REFERENCE_SYMBOLS) == set(symbols)
+    if hdr == "ours":
+        assert set(symbols) <= _declared("fourier.h")
+    prog = tmp_path / ("refs.c" if cc == "gcc" else "refs.cpp")
+    prog.write_text("#ifdef __cplusplus\nextern \"C\" {\n#endif\n"
+                    + "".join(f"void {s}(void);\n" for s in symbols)
+                    + "#ifdef __cplusplus\n}\n#endif\n"
+                    + "int main(void) {\n  void (*volatile refs[])(void) = {" + ", ".join(symbols) + "};\n"
+                    + "  return refs[0] == 0;\n}\n")
     exe = tmp_path / "ref_test"
-    cmd = [cc, "-Wall", "-Wextra", "-pedantic", "-Werror", "-I", inc,
-           os.path.join("/root/reference/fourier-ffi", src), "-o", str(exe), "-L", LIBDIR, "-lfourier", "-lm"]
-    subprocess.run(cmd, check=True, capture_output=True)
+    cmd = [cc, "-Wall", "-Wextra", "-pedantic", "-Werror", str(prog), "-o", str(exe), "-L", LIBDIR, "-lfourier", "-lm"]
+    r = subprocess.run(cmd, capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_transform_enum_mirrors_reference():

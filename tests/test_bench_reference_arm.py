@@ -28,3 +28,25 @@ def test_reference_arm_prints_one_contract_line():
     import bench
     n, batch, real, desc = bench.WORKLOADS["c1"]
     assert rec["config"] == bench.workload_config(desc, n, batch, 1, real)
+
+
+def test_reference_arm_dumps_its_last_step(tmp_path):
+    """--dump-outputs: the transforms of the last timed step as float32 (real, imaginary) pairs, and their indices."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    from oracle import oracle as O
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "c1",
+                        "--steps", "1", "--warmup", "0", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    rec = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+    assert rec["dump"]["files"] == ["output.npy", "output_rows.npy"]
+    y, rows = np.load(out / "output.npy"), np.load(out / "output_rows.npy")
+    assert y.dtype == np.float32 and rows.dtype == np.float64 and y.shape[1:] == (1024, 2)
+    assert y.shape[0] == rows.shape[0] == rec["dump"]["rows"] and y.nbytes + rows.nbytes <= 64 << 20
+    assert np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < rec["dump"]["of_rows"]
+    got = y[..., 0] + 1j * y[..., 1]
+    x = np.concatenate([O.fill_input(1, 1024, np.complex64, first_transform=int(row)) for row in rows])
+    want = O.transform(x, O.FFT)
+    assert np.abs(got - want).max() / np.abs(want).max() < 1e-5
