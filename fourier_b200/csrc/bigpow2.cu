@@ -8,23 +8,12 @@
 //   and without any table of N entries (the reference's twiddle table, autosort/mod.rs:24-46, would be 128 MB per
 //   direction at N = 2^24; the general per-stage path of this library needs one too).
 #include <algorithm>
-#include <cmath>
-#include <cstdlib>
 
 #include "outer_kernels.cuh"
 #include "plan.h"
 #include "twopass_kernels.cuh"
 
 namespace fb200 {
-
-#define FB_CHECK(expr)                                                                       \
-  do {                                                                                       \
-    cudaError_t _e = (expr);                                                                 \
-    if (_e != cudaSuccess) {                                                                 \
-      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
-      return _e;                                                                             \
-    }                                                                                        \
-  } while (0)
 
 namespace {
 
@@ -116,7 +105,7 @@ cudaError_t Plan<T>::init_threepass_radix3() {
   int b = 1;
   while (r % 3 == 0 && b < 27) { r /= 3; b *= 3; }
   if (b == 1 || (r & (r - 1)) || r % 3 == 0) return cudaErrorNotSupported;
-  inner_.reset(Plan<T>::create(r, device_, true));
+  inner_.reset(Plan<T>::create(r, device_, true, tuning_));
   if (!inner_ || inner_->path() != Path::kTwoPass) { inner_.reset(); return cudaErrorNotSupported; }
   n1_ = (size_t)b;
   n2_ = r;
@@ -133,14 +122,14 @@ cudaError_t Plan<T>::init_bigpow2() {
   if (((size_t)1 << k) != n_ || k < k_min || k > k_max) return cudaErrorNotSupported;
   // rows of 2^14 where possible (the best tile-kernel size with 16-row tiles), the outer pass takes the rest
   int a = std::min(a_max, std::max(a_min, k - 14));
-  if (const char* env = std::getenv("FOURIER_B200_BIG_NA")) a = std::min(a_max, std::max(a_min, atoi(env)));
+  if (tuning_.big_na) a = std::min(a_max, std::max(a_min, *tuning_.big_na));
   const ColumnOps<T>* col = column_lookup<T>(a);
   if (!col) return cudaErrorNotSupported;
-  inner_.reset(Plan<T>::create((size_t)1 << (k - a), device_, true));
+  inner_.reset(Plan<T>::create((size_t)1 << (k - a), device_, true, tuning_));
   if (!inner_ || inner_->path() != Path::kTwoPass) { inner_.reset(); return cudaErrorNotSupported; }
   n1_ = (size_t)1 << a;
   n2_ = (size_t)1 << (k - a);
-  FB_CHECK((twopass::upload_vec<T, TwPair<T>>(tw_a_, twopass::make_twa<T>(col->ra, col->rb))));
+  FB_CHECK(upload(tw_a_, twopass::make_twa<T>(col->ra, col->rb)));
   fast_ops_ = col;
   return cudaSuccess;
 }
@@ -149,9 +138,7 @@ template <typename T>
 cudaError_t Plan<T>::exec_bigpow2(const C* in, C* out, size_t batch, int code, cudaStream_t s) {
   const auto* col = static_cast<const ColumnOps<T>*>(fast_ops_);   // nullptr with an outer radix-3 pass
   const bool fwd = transform_is_forward(code);
-  T scale = (T)1;
-  if (code == kIfft) scale = (T)1 / (T)n_;
-  else if (code == kSqrtScaledFft || code == kSqrtScaledIfft) scale = (T)1 / std::sqrt((T)n_);
+  const T scale = scale_for<T>(code, n_);
   // the intermediate A[ka][nb] of a few transforms at a time (at most 2 GB of scratch, at least one transform)
   const size_t chunk = std::min(batch, std::max<size_t>(1, ((size_t)2 << 30) / (n_ * sizeof(C))));
   // the row kernel works on whole tiles of up to 32 rows: 3 / 9 / 27 rows per transform are padded up (the padding rows

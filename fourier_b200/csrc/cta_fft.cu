@@ -10,15 +10,6 @@
 
 namespace fb200 {
 
-#define FB_CHECK(expr)                                                                       \
-  do {                                                                                       \
-    cudaError_t _e = (expr);                                                                 \
-    if (_e != cudaSuccess) {                                                                 \
-      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
-      return _e;                                                                             \
-    }                                                                                        \
-  } while (0)
-
 namespace {
 
 constexpr size_t kSmemLimit = 227 * 1024;
@@ -52,36 +43,16 @@ template <typename T> int group_for(int len) {
 template <typename T, bool DIR, bool CHIRP>
 cudaError_t launch(const cta::Args<T>& a, int sms, cudaStream_t s) {
   const size_t bytes = smem_bytes<T>(a.group, a.len);
-  static size_t configured = 0;   // per instantiation
-  if (bytes > configured) {
-    cudaError_t e = cudaFuncSetAttribute(cta::cta_fft_kernel<T, DIR, CHIRP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)kSmemLimit);
-    if (e != cudaSuccess) return e;
-    // several CTAs per SM need the full shared-memory carve-out (the default heuristic left room for two of three)
-    e = cudaFuncSetAttribute(cta::cta_fft_kernel<T, DIR, CHIRP>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                             (int)cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    configured = kSmemLimit;
-  }
+  // several CTAs per SM need the full shared-memory carve-out (the default heuristic left room for two of three)
+  static std::atomic<unsigned long long> prepared{0};
+  if (cudaError_t e = ensure_dynamic_smem(cta::cta_fft_kernel<T, DIR, CHIRP>, kSmemLimit, prepared,
+                                          (int)cudaSharedmemCarveoutMaxShared))
+    return e;
   const size_t groups = ((size_t)a.batch + a.group - 1) / a.group;
   const size_t per_sm = std::max<size_t>(1, std::min<size_t>(8, kSmemLimit / (bytes + 1024)));
   const unsigned grid = (unsigned)std::min<size_t>(groups, (size_t)sms * per_sm);
   cta::cta_fft_kernel<T, DIR, CHIRP><<<grid, cta::kThreads, bytes, s>>>(a);
   return cudaGetLastError();
-}
-
-template <typename T>
-cudaError_t upload(DeviceBuffer& buf, const std::vector<cpx<T>>& host) {
-  cudaError_t e = buf.reserve(std::max<size_t>(host.size(), 1) * sizeof(cpx<T>));
-  if (e != cudaSuccess) return e;
-  return cudaMemcpy(buf.data(), host.data(), host.size() * sizeof(cpx<T>), cudaMemcpyHostToDevice);
-}
-
-int sm_count() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
 }
 
 }  // namespace
@@ -104,8 +75,7 @@ cudaError_t Plan<T>::init_cta(size_t len) {
   cta::Stages st;
   if (!cta::factorize(len, st)) return cudaErrorNotSupported;
   radices_.assign(st.radix, st.radix + st.count);
-  FB_CHECK(upload<T>(wtab_, cta::make_stage_twiddles<T>(len, st, host_twiddle)));
-  sm_count_ = sm_count();
+  FB_CHECK(upload(wtab_, cta::make_stage_twiddles<T>(len, st, host_twiddle)));
   return cudaSuccess;
 }
 
@@ -121,9 +91,7 @@ cudaError_t Plan<T>::exec_cta(const C* in, C* out, size_t batch, int code, cudaS
   a.n = (int)n_;
   a.len = (int)cta_len_;
   a.group = group_for<T>(a.len);
-  T scale = (T)1;
-  if (code == kIfft) scale = (T)1 / (T)n_;
-  else if (code == kSqrtScaledFft || code == kSqrtScaledIfft) scale = (T)1 / std::sqrt((T)n_);
+  T scale = scale_for<T>(code, n_);
   if (chirp) scale /= (T)cta_len_;      // the unscaled inner inverse transform
   a.scale = scale;
   cta::factorize(cta_len_, a.st);

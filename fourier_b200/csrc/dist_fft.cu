@@ -4,7 +4,6 @@
 // plan-owned ones (lanes), each with its own intermediate, so that pass 1 of one chunk (HBM reads, no NVLink
 // traffic) runs beside pass 2 of another (NVLink stores).
 #include <algorithm>
-#include <cstdlib>
 #include <type_traits>
 
 #include "dist_kernels.cuh"
@@ -12,15 +11,6 @@
 #include "twopass_kernels.cuh"
 
 namespace fb200 {
-
-#define FB_CHECK(expr)                                                                       \
-  do {                                                                                       \
-    cudaError_t _e = (expr);                                                                 \
-    if (_e != cudaSuccess) {                                                                 \
-      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
-      return _e;                                                                             \
-    }                                                                                        \
-  } while (0)
 
 namespace {
 
@@ -33,7 +23,8 @@ template <typename T> struct RowsExchangeCall {
 // Tiles of twice as many transforms where the configuration's pass-2 tile has 16 (f32) / 8 (f64): a warp's store is then
 // one 256-byte run instead of two 128-byte pieces.  Measured (profiles/r02_rows_exchange_knobs.txt, r02_c5_modes_8gpu.json):
 // N = 2^30 on 2 GPUs 12.64 -> 12.27 ms, on 8 GPUs 5.13 -> 5.15 ms (no change), one GPU (three-pass path) no change.
-// Paddings are the bank-conflict-free ones (tools/emulate.cu).  FOURIER_B200_DIST_WIDE=0 selects the narrow tiles.
+// Paddings are the bank-conflict-free ones (tools/emulate.cu).  The narrow tiles remain for row counts that are not a
+// multiple of the wide tile.
 template <class S, typename T> struct WideShape { using type = S; };
 template <> struct WideShape<twopass::Shape<8, 16, 16, 16, 2>, float> { using type = twopass::Shape<8, 16, 16, 32, 2>; };
 template <> struct WideShape<twopass::Shape<16, 16, 16, 16, 1>, float> { using type = twopass::Shape<16, 16, 16, 32, 1>; };
@@ -76,10 +67,6 @@ template <class G, bool WIDE, typename T> cudaError_t dispatch_rows_exchange(con
   if (c.fwd) return c.twiddle ? launch_rows_exchange<G, true, 1, MORE, WIDE>(c) : launch_rows_exchange<G, true, 0, MORE, WIDE>(c);
   return c.twiddle ? launch_rows_exchange<G, false, 2, MORE, WIDE>(c) : launch_rows_exchange<G, false, 0, MORE, WIDE>(c);
 }
-bool wide_wanted() {
-  static const bool w = [] { const char* e = std::getenv("FOURIER_B200_DIST_WIDE"); return !e || atoi(e) != 0; }();
-  return w;
-}
 
 }  // namespace
 
@@ -116,7 +103,7 @@ cudaError_t Plan<T>::exec_rows_exchange(const C* in, size_t rows, bool forward, 
     c2 = decltype(g)::C2;
     c2w = ExchangeTile<decltype(g), true, T>::C;
   });
-  const bool wide = wide_wanted() && c2w != c2 && rows % (size_t)c2w == 0;
+  const bool wide = c2w != c2 && rows % (size_t)c2w == 0;
   if (wide) c2 = c2w;
   if (c2 == 0 || rows % (size_t)c2) {
     set_last_error("rows_exchange: the number of rows must be a multiple of " + std::to_string(c2));
@@ -127,17 +114,11 @@ cudaError_t Plan<T>::exec_rows_exchange(const C* in, size_t rows, bool forward, 
   while (((size_t)1 << cb_shift) < n_ / (size_t)nranks) ++cb_shift;
   // chunks of whole tiles, two of them in flight.  Measured on 2 B200s (N = 2^28, profiles/r02_c5_fused_ab_2gpu.txt):
   // 16 MB chunks 3.60 ms per transform, 32 MB 3.23, 64 MB 3.07 -- NVLink, not the L2 residency of the intermediate,
-  // bounds this path, and longer kernels overlap better across the two streams.  FOURIER_B200_DIST_CHUNK_MB overrides.
-  size_t mb = 64;
-  if (const char* e = std::getenv("FOURIER_B200_DIST_CHUNK_MB")) mb = (size_t)std::max(1, atoi(e));
-  else if (const char* e2 = std::getenv("FOURIER_B200_CHUNK_MB")) mb = (size_t)std::max(1, atoi(e2));
-  const size_t want = std::max<size_t>(1, (mb << 20) / (n_ * sizeof(C)));
+  // bounds this path, and longer kernels overlap better across the two streams (tuning_.dist_chunk_mb, 64 by default).
+  const size_t want = std::max<size_t>(1, (tuning_.dist_chunk_mb << 20) / (n_ * sizeof(C)));
   size_t chunk = std::max<size_t>((size_t)c2, std::min(want, rows) / (size_t)c2 * (size_t)c2);
   // lanes: chunks rotate over the caller's stream and up to three plan-owned ones, each with its own intermediate
-  int nlanes = 2;
-  if (const char* env = std::getenv("FOURIER_B200_DIST_LANES")) nlanes = std::min(4, std::max(1, atoi(env)));
-  if (const char* env = std::getenv("FOURIER_B200_DIST_OVERLAP")) { if (atoi(env) == 0) nlanes = 1; }
-  nlanes = (int)std::min<size_t>((size_t)nlanes, (rows + chunk - 1) / chunk);
+  const int nlanes = (int)std::min<size_t>((size_t)tuning_.dist_lanes, (rows + chunk - 1) / chunk);
   FB_CHECK(work_.reserve((size_t)nlanes * chunk * n_ * sizeof(C)));
   cudaStream_t lanes[4] = {s, s, s, s};
   if (nlanes > 1) {

@@ -72,11 +72,6 @@ exchange_kernel(const cpx<T>* __restrict__ in, PeerPtrs outs, int nranks, int me
   }
 }
 
-int env_blocks() {
-  const char* e = std::getenv("FOURIER_B200_EXCHANGE_BLOCKS");
-  return e ? atoi(e) : 0;
-}
-
 }  // namespace
 
 template <typename T>
@@ -97,8 +92,11 @@ cudaError_t launch_exchange(const cpx<T>* in, void* const* outs, int nranks, int
   PeerPtrs p;
   for (int i = 0; i < kMaxPeers; ++i) p.p[i] = i < nranks ? outs[i] : nullptr;
   const unsigned total = (unsigned)(tiles_c * tiles_r * (size_t)nranks);
-  // FOURIER_B200_EXCHANGE_BLOCKS=n (experiment, not yet measured): n persistent blocks instead of one block per tile
-  const int limit = env_blocks();
+  // FOURIER_B200_EXCHANGE_BLOCKS=n (experiment, not yet measured): n persistent blocks instead of one block per tile.
+  // Unlike the plans' knobs (Tuning) this one is read on every call: the exchange has no plan to hold it, and callers
+  // switch it between calls.
+  const char* blocks = env_value("FOURIER_B200_EXCHANGE_BLOCKS");
+  const int limit = blocks ? atoi(blocks) : 0;
 #define FB_EXCHANGE_LAUNCH(TW)                                                                                      \
   do {                                                                                                               \
     if (limit > 0 && (unsigned)limit < total)                                                                        \

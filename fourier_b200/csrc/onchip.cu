@@ -3,23 +3,12 @@
 // Reference counterparts: Autosort for small sizes (autosort/mod.rs:141-166) and
 // Bluesteins::transform_in_place / apply (bluesteins.rs:193-259).
 #include <algorithm>
-#include <cmath>
-#include <cstdlib>
 
 #include "onchip_kernels.cuh"
 #include "plan.h"
 #include "tables.cuh"  // make_twa
 
 namespace fb200 {
-
-#define FB_CHECK(expr)                                                                       \
-  do {                                                                                       \
-    cudaError_t _e = (expr);                                                                 \
-    if (_e != cudaSuccess) {                                                                 \
-      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
-      return _e;                                                                             \
-    }                                                                                        \
-  } while (0)
 
 namespace {
 
@@ -100,10 +89,7 @@ template <> const OnChipOps<float>* onchip_lookup<float>(size_t l) {
     case 512: return OnChipImpl<float, 16, 32, 32, 8, 2, 8>::ops();
     case 1024:
       // The fused Bluestein kernel parks the even half in thread-local memory (16 warps per SM, measured
-      // 1.16e11 samples/s at N=1009); FOURIER_B200_BLUESTEIN_LOCAL=0 selects the shared-memory stash
-      // (11 warps per SM, 1.01e11).
-      if (const char* e = std::getenv("FOURIER_B200_BLUESTEIN_LOCAL"); e && atoi(e) == 0)
-        return OnChipImpl<float, 32, 32, 32, 8, 2, 11>::ops();
+      // 1.16e11 samples/s at N=1009); the shared-memory stash (11 warps per SM) measured 1.01e11.
       return OnChipImpl<float, 32, 32, 32, 8, 2, 16, true>::ops();
     default: return nullptr;
   }
@@ -117,20 +103,6 @@ template <> const OnChipOps<double>* onchip_lookup<double>(size_t l) {
   }
 }
 
-template <typename T, typename U>
-cudaError_t upload_vec(DeviceBuffer& buf, const std::vector<U>& host) {
-  cudaError_t e = buf.reserve(host.size() * sizeof(U));
-  if (e != cudaSuccess) return e;
-  return cudaMemcpy(buf.data(), host.data(), host.size() * sizeof(U), cudaMemcpyHostToDevice);
-}
-
-int sm_count() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
-}
-
 }  // namespace
 
 template <typename T>
@@ -138,9 +110,8 @@ cudaError_t Plan<T>::init_onchip() {
   const OnChipOps<T>* ops = onchip_lookup<T>(n_);
   if (!ops) return cudaErrorNotSupported;
   FB_CHECK(ops->prepare());
-  FB_CHECK((upload_vec<T, TwPair<T>>(tw_a_, twopass::make_twa<T>(ops->ra, ops->rb))));
+  FB_CHECK(upload(tw_a_, twopass::make_twa<T>(ops->ra, ops->rb)));
   fast_ops_ = ops;
-  sm_count_ = sm_count();
   return cudaSuccess;
 }
 
@@ -149,9 +120,7 @@ cudaError_t Plan<T>::exec_onchip(const C* in, C* out, size_t batch, int code, cu
   const auto* ops = static_cast<const OnChipOps<T>*>(fast_ops_);
   const bool fwd = transform_is_forward(code);
   const bool do_scale = !(code == kFft || code == kUnscaledIfft);
-  T scale = (T)1;
-  if (code == kIfft) scale = (T)1 / (T)n_;
-  else if (do_scale) scale = (T)1 / std::sqrt((T)n_);
+  const T scale = scale_for<T>(code, n_);
   FB_CHECK(ops->fft(in, out, tw_a_.data(), batch, fwd, scale, do_scale, sm_count_, s));
   launches_ += 1;
   return cudaSuccess;
@@ -166,7 +135,7 @@ cudaError_t Plan<T>::init_bluestein_fused(const std::vector<double>& chirp_re, c
   const OnChipOps<T>* ops = onchip_lookup<T>(l);
   if (!ops || !ops->bluestein) return cudaErrorNotSupported;
   FB_CHECK(ops->prepare());
-  FB_CHECK((upload_vec<T, TwPair<T>>(tw_a_, twopass::make_twa<T>(ops->ra, ops->rb))));
+  FB_CHECK(upload(tw_a_, twopass::make_twa<T>(ops->ra, ops->rb)));
   // layout per direction d (0 forward, 1 inverse): [chirp | wm | wce | wco], L entries each
   std::vector<cpx<T>> tab(2 * 4 * l, mk<T>((T)0, (T)0));
   for (int d = 0; d < 2; ++d) {
@@ -181,9 +150,8 @@ cudaError_t Plan<T>::init_bluestein_fused(const std::vector<double>& chirp_re, c
       t[3 * l + i] = mk<T>((T)w_re[2 * i + 1], (T)(-sgn * w_im[2 * i + 1]));  // conj(W_dir[2k+1])
     }
   }
-  FB_CHECK((upload_vec<T, cpx<T>>(tbase_, tab)));
+  FB_CHECK(upload(tbase_, tab));
   fast_ops_ = ops;
-  sm_count_ = sm_count();
   return cudaSuccess;
 }
 
@@ -191,10 +159,7 @@ template <typename T>
 cudaError_t Plan<T>::exec_bluestein_fused(const C* in, C* out, size_t batch, int code, cudaStream_t s) {
   const auto* ops = static_cast<const OnChipOps<T>*>(fast_ops_);
   const bool fwd = transform_is_forward(code);
-  T scale = (T)1;
-  if (code == kIfft) scale = (T)1 / (T)n_;
-  else if (code == kSqrtScaledFft || code == kSqrtScaledIfft) scale = (T)1 / std::sqrt((T)n_);
-  scale /= (T)m_;
+  const T scale = scale_for<T>(code, n_) / (T)m_;
   const size_t l = m_ / 2;
   const C* t = (const C*)tbase_.data() + (fwd ? 0 : 4 * l);
   FB_CHECK(ops->bluestein(in, out, tw_a_.data(), t, t + l, t + 2 * l, t + 3 * l, n_, batch, scale, sm_count_, s));

@@ -23,15 +23,6 @@ static thread_local std::string g_last_error;
 void set_last_error(const std::string& s) { g_last_error = s; }
 const char* last_error() { return g_last_error.c_str(); }
 
-#define FB_CHECK(expr)                                                                       \
-  do {                                                                                       \
-    cudaError_t _e = (expr);                                                                 \
-    if (_e != cudaSuccess) {                                                                 \
-      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
-      return _e;                                                                             \
-    }                                                                                        \
-  } while (0)
-
 const char* path_name(Path p) {
   switch (p) {
     case Path::kTrivial: return "trivial";
@@ -62,6 +53,31 @@ size_t bluestein_inner_size(size_t n) {
   return m;
 }
 
+const char* env_value(const char* name) { return std::getenv(name); }
+
+Tuning Tuning::from_env() {
+  auto env_int = [](const char* name) -> std::optional<int> {
+    const char* e = env_value(name);
+    if (!e) return std::nullopt;
+    return atoi(e);
+  };
+  Tuning t;
+  if (auto v = env_int("FOURIER_B200_TWOPASS"); v && *v == 0) t.twopass = false;
+  if (auto v = env_int("FOURIER_B200_FUSED"); v && *v == 0) t.fused = false;
+  t.ring = env_int("FOURIER_B200_RING");
+  t.lag = env_int("FOURIER_B200_LAG");
+  const auto chunk_mb = env_int("FOURIER_B200_CHUNK_MB");
+  if (chunk_mb) t.chunk_mb = (size_t)std::max(1, *chunk_mb);
+  if (auto v = env_int("FOURIER_B200_DIST_CHUNK_MB")) t.dist_chunk_mb = (size_t)std::max(1, *v);
+  else if (chunk_mb) t.dist_chunk_mb = t.chunk_mb;
+  if (auto v = env_int("FOURIER_B200_DIST_LANES")) t.dist_lanes = std::min(4, std::max(1, *v));
+  if (auto v = env_int("FOURIER_B200_DIST_OVERLAP"); v && *v == 0) t.dist_lanes = 1;
+  t.big_na = env_int("FOURIER_B200_BIG_NA");
+  t.zero_copy = env_value("FOURIER_B200_NO_ZEROCOPY") == nullptr;
+  if (const char* e = env_value("FOURIER_B200_TRACE")) t.trace = e;
+  return t;
+}
+
 DeviceBuffer::~DeviceBuffer() { release(); }
 void DeviceBuffer::release() {
   if (ptr_) cudaFree(ptr_);
@@ -79,24 +95,6 @@ cudaError_t DeviceBuffer::reserve(size_t bytes) {
 
 namespace {
 
-template <typename T>
-cudaError_t upload(DeviceBuffer& buf, const std::vector<cpx<T>>& host) {
-  cudaError_t e = buf.reserve(std::max<size_t>(host.size(), 1) * sizeof(cpx<T>));
-  if (e != cudaSuccess) return e;
-  if (host.empty()) return cudaSuccess;
-  return cudaMemcpy(buf.data(), host.data(), host.size() * sizeof(cpx<T>), cudaMemcpyHostToDevice);
-}
-
-// Scale factor of a Transform code for length n (autosort/mod.rs:381-385, bluesteins.rs:240-258).
-template <typename T> T scale_for(int code, size_t n) {
-  switch (code) {
-    case kIfft: return (T)1 / (T)n;
-    case kSqrtScaledFft:
-    case kSqrtScaledIfft: return (T)1 / std::sqrt((T)n);
-    default: return (T)1;
-  }
-}
-
 constexpr size_t kScratchTargetBytes = (size_t)512 << 20;  // per scratch buffer on the general path
 constexpr size_t kHostChunkBytes = (size_t)64 << 20;       // host-pointer pipeline granule
 constexpr size_t kHostSmallBytes = (size_t)1 << 20;        // below this a host call takes the single-stream latency path
@@ -109,12 +107,18 @@ constexpr size_t kHostZeroCopyBytes = (size_t)64 << 10;    // below this the ker
 // ---------------------------------------------------------------------------------------------------
 template <typename T>
 Plan<T>* Plan<T>::create(size_t n, int device, bool allow_fast_paths) {
+  return create(n, device, allow_fast_paths, Tuning::from_env());
+}
+
+template <typename T>
+Plan<T>* Plan<T>::create(size_t n, int device, bool allow_fast_paths, const Tuning& tuning) {
   if (n == 0) {
     set_last_error("size 0 is not a valid transform length");
     return nullptr;
   }
   Plan<T>* p = new (std::nothrow) Plan<T>();
   if (!p) return nullptr;
+  p->tuning_ = tuning;
   cudaError_t e = cudaErrorUnknown;
   try {
     e = p->init(n, device, allow_fast_paths);
@@ -162,23 +166,23 @@ cudaError_t Plan<T>::init(size_t n, int device, bool allow_fast_paths) {
   device_ = device;
   DeviceGuard g(device_);
   if (!g.ok) { set_last_error("cudaSetDevice failed"); return cudaErrorInvalidDevice; }
+  if (cudaDeviceGetAttribute(&sm_count_, cudaDevAttrMultiProcessorCount, device_) != cudaSuccess) sm_count_ = 148;
   if (n == 1) { path_ = Path::kTrivial; return cudaSuccess; }
   if (is_23_smooth(n)) {
     const bool pow2 = (n & (n - 1)) == 0;
     if (allow_fast_paths && pow2) {
       if (init_onchip() == cudaSuccess) { path_ = Path::kOnChip; return cudaSuccess; }
-      // FOURIER_B200_TWOPASS=0 (experiment knob): skip the two-pass kernels, so that sizes the CTA kernel also
+      // tuning_.twopass = false (experiment knob): skip the two-pass kernels, so that sizes the CTA kernel also
       // covers can be measured on it
-      const char* tp = std::getenv("FOURIER_B200_TWOPASS");
-      if (!(tp && atoi(tp) == 0) && init_twopass() == cudaSuccess) { path_ = Path::kTwoPass; return cudaSuccess; }
+      if (tuning_.twopass && init_twopass() == cudaSuccess) { path_ = Path::kTwoPass; return cudaSuccess; }
       // beyond the two-pass sizes: an outer column pass around two-pass rows (bigpow2.cu)
-      if (!(tp && atoi(tp) == 0) && init_bigpow2() == cudaSuccess) { path_ = Path::kThreePass; return cudaSuccess; }
+      if (tuning_.twopass && init_bigpow2() == cudaSuccess) { path_ = Path::kThreePass; return cudaSuccess; }
     }
     // everything else that fits two shared-memory buffers: one kernel, one HBM round trip
     if (allow_fast_paths && init_cta(n) == cudaSuccess) { path_ = Path::kCta; return cudaSuccess; }
-    // 3^b * 2^k (b <= 3) with a two-pass power of two: outer radix-3^b pass + two-pass rows (bigpow2.cu)
-    const char* tp3 = std::getenv("FOURIER_B200_TWOPASS");   // =0 (experiment knob): measure the per-stage path instead
-    if (allow_fast_paths && !pow2 && !(tp3 && atoi(tp3) == 0) && init_threepass_radix3() == cudaSuccess) {
+    // 3^b * 2^k (b <= 3) with a two-pass power of two: outer radix-3^b pass + two-pass rows (bigpow2.cu); without
+    // tuning_.twopass the per-stage path is measured instead
+    if (allow_fast_paths && !pow2 && tuning_.twopass && init_threepass_radix3() == cudaSuccess) {
       path_ = Path::kThreePass;
       return cudaSuccess;
     }
@@ -209,7 +213,7 @@ cudaError_t Plan<T>::init_global_stages() {
     host_twiddle(k, n_, &re, &im);
     w[k] = mk<T>((T)re, (T)im);
   }
-  FB_CHECK(upload<T>(wtab_, w));
+  FB_CHECK(upload(wtab_, w));
   return cudaSuccess;
 }
 
@@ -243,16 +247,16 @@ cudaError_t Plan<T>::init_bluestein(bool allow_fast_paths) {
   }
   if (allow_fast_paths && init_cta(m_) == cudaSuccess) {
     // inner size above the warp-level kernel: the CTA-level kernel in chirp mode, still one launch
-    FB_CHECK(upload<T>(chirp_, chirp));
-    FB_CHECK(upload<T>(wf_, wf));
+    FB_CHECK(upload(chirp_, chirp));
+    FB_CHECK(upload(wf_, wf));
     cta_chirp_ = true;
     path_ = Path::kBluesteinFused;
     return cudaSuccess;
   }
-  inner_.reset(Plan<T>::create(m_, device_, allow_fast_paths));
+  inner_.reset(Plan<T>::create(m_, device_, allow_fast_paths, tuning_));
   if (!inner_) return cudaErrorUnknown;
-  FB_CHECK(upload<T>(chirp_, chirp));
-  FB_CHECK(upload<T>(wf_, wf));
+  FB_CHECK(upload(chirp_, chirp));
+  FB_CHECK(upload(wf_, wf));
   path_ = Path::kBluestein;
   return cudaSuccess;
 }
@@ -380,7 +384,7 @@ cudaError_t Plan<T>::exec_host(const C* in, C* out, size_t batch, int code) {
     // Latency path (the reference ABI's single small transform, fourier-ffi/src/lib.rs:46-59): nothing to
     // pipeline, so one stream, no events, one synchronisation: H2D, kernel(s), D2H back to back.
     cudaStream_t s = streams_[1];
-    if (batch * bytes_per <= kHostZeroCopyBytes && !std::getenv("FOURIER_B200_NO_ZEROCOPY")) {
+    if (batch * bytes_per <= kHostZeroCopyBytes && tuning_.zero_copy) {
       // Smallest calls: the two DMA copies cost more than the transform.  The kernels read the input from and write
       // the result to a pinned, device-mapped bounce buffer over PCIe themselves (one launch, one synchronisation;
       // the CPU copies 2 x <= 64 KB).  Measured: 24 -> ~12 us per 1024-point call (profiles/r02_latency.txt).

@@ -9,15 +9,31 @@
 
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstddef>
 #include <memory>
+#include <optional>
 #include <string>
 #include <vector>
 
 #include "cplx.cuh"
 
 namespace fb200 {
+
+// thread-local error text for the C ABI
+void set_last_error(const std::string& s);
+const char* last_error();
+
+#define FB_CHECK(expr)                                                                       \
+  do {                                                                                       \
+    cudaError_t _e = (expr);                                                                 \
+    if (_e != cudaSuccess) {                                                                 \
+      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
+      return _e;                                                                             \
+    }                                                                                        \
+  } while (0)
 
 // Execution strategy chosen at plan time.
 enum class Path : int {
@@ -56,18 +72,51 @@ struct DeviceGuard {
 };
 
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is a per-device setting: done once per kernel AND device (a process
-// may hold plans on several GPUs).  `done` is the kernel's own bit mask of prepared devices.
+// may hold plans on several GPUs).  `done` is the kernel's own bit mask of prepared devices.  carveout >= 0 also sets
+// the preferred shared-memory carve-out (a cudaSharedmemCarveout value or a percentage).
 template <class Kernel>
-inline cudaError_t ensure_dynamic_smem(Kernel kernel, size_t bytes, std::atomic<unsigned long long>& done) {
+inline cudaError_t ensure_dynamic_smem(Kernel kernel, size_t bytes, std::atomic<unsigned long long>& done,
+                                       int carveout = -1) {
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
   const unsigned long long bit = 1ull << (dev & 63);
   if (done.load(std::memory_order_acquire) & bit) return cudaSuccess;
   e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess && carveout >= 0)
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
   if (e == cudaSuccess) done.fetch_or(bit, std::memory_order_release);
   return e;
 }
+
+// Scale factor of a Transform code for length n (autosort/mod.rs:381-385, bluesteins.rs:240-258).
+template <typename T> T scale_for(int code, size_t n) {
+  switch (code) {
+    case kIfft: return (T)1 / (T)n;
+    case kSqrtScaledFft:
+    case kSqrtScaledIfft: return (T)1 / std::sqrt((T)n);
+    default: return (T)1;
+  }
+}
+
+// The library's one environment lookup: the value of variable `name`, nullptr when it is unset.
+const char* env_value(const char* name);
+
+// Experiment knobs (FOURIER_B200_* environment variables).  A plan reads them once, when it is created, and hands the
+// same values to its inner plans, so that a plan and its exec calls never see two configurations.
+struct Tuning {
+  bool twopass = true;          // TWOPASS=0: skip the two-pass, three-pass and radix-3 three-pass paths
+  bool fused = true;            // FUSED=0: the two tile kernels instead of the persistent kernel
+  std::optional<int> ring, lag; // RING, LAG: staging ring of the persistent kernel; unset = the configuration's own
+  size_t chunk_mb = 32;         // CHUNK_MB: L2-resident chunk of the two-pass tile kernels
+  size_t dist_chunk_mb = 64;    // DIST_CHUNK_MB, else CHUNK_MB: chunk of the fused row FFT + exchange
+  int dist_lanes = 2;           // DIST_LANES (1 .. 4), DIST_OVERLAP=0 forces 1: streams the chunks rotate over
+  std::optional<int> big_na;    // BIG_NA: log2 of the outer pass length of the three-pass path
+  bool zero_copy = true;        // NO_ZEROCOPY (set): the smallest host calls take the copy path
+  std::string trace;            // TRACE=<file>: phase timeline of the persistent kernel, written after every call
+
+  static Tuning from_env();
+};
 
 // Grow-only device allocation.
 class DeviceBuffer {
@@ -86,6 +135,15 @@ class DeviceBuffer {
   size_t bytes_ = 0;
 };
 
+// Copies a host table into `buf`, grown as needed (an empty table still reserves one element).
+template <typename U>
+cudaError_t upload(DeviceBuffer& buf, const std::vector<U>& host) {
+  cudaError_t e = buf.reserve(std::max<size_t>(host.size(), 1) * sizeof(U));
+  if (e != cudaSuccess) return e;
+  if (host.empty()) return cudaSuccess;
+  return cudaMemcpy(buf.data(), host.data(), host.size() * sizeof(U), cudaMemcpyHostToDevice);
+}
+
 struct PlanInfo {
   size_t size = 0;
   int path = 0;
@@ -103,7 +161,7 @@ class Plan {
   using C = cpx<T>;
 
   // Returns nullptr (and sets last_error) when the plan cannot be built; size 0 is refused
-  // (the reference never returns for 0: autosort/mod.rs:112).
+  // (the reference never returns for 0: autosort/mod.rs:112).  The Tuning knobs are read from the environment here.
   static Plan* create(size_t n, int device, bool allow_fast_paths = true);
   ~Plan();
 
@@ -140,6 +198,8 @@ class Plan {
 
  private:
   Plan() = default;
+  // inner plans (three-pass rows, Bluestein inner transform) take their parent's knobs
+  static Plan* create(size_t n, int device, bool allow_fast_paths, const Tuning& tuning);
   cudaError_t init(size_t n, int device, bool allow_fast_paths);
 
   cudaError_t exec_global_stages(const C* in, C* out, size_t batch, int code, cudaStream_t s);
@@ -164,6 +224,7 @@ class Plan {
   int device_ = 0;
   Path path_ = Path::kTrivial;
   unsigned long long launches_ = 0;
+  Tuning tuning_;
 
   // kGlobalStages: radices of the Stockham stages and the full forward table w_N^k, k < N
   std::vector<int> radices_;
@@ -198,10 +259,6 @@ class Plan {
   void* zc_in_ = nullptr;         // pinned, device-mapped bounce buffers of the smallest host calls (64 KB each)
   void* zc_out_ = nullptr;
 };
-
-// thread-local error text for the C ABI
-void set_last_error(const std::string& s);
-const char* last_error();
 
 // ---- kernel launchers implemented in the .cu files ------------------------------------------------
 

@@ -14,22 +14,12 @@
 //   pass 1 reads  x  as C consecutive columns (C*8 B per row),  writes A[k1][n2] the same way;
 //   pass 2 reads  A  as whole contiguous rows,                  writes X as C consecutive k1.
 #include <cstdio>
-#include <cstdlib>
 
 #include "plan.h"
 #include "fused_kernels.cuh"
 #include "twopass_kernels.cuh"
 
 namespace fb200 {
-
-#define FB_CHECK(expr)                                                                       \
-  do {                                                                                       \
-    cudaError_t _e = (expr);                                                                 \
-    if (_e != cudaSuccess) {                                                                 \
-      set_last_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                    \
-      return _e;                                                                             \
-    }                                                                                        \
-  } while (0)
 
 using namespace twopass;
 
@@ -49,11 +39,6 @@ EncodeTiledFn encode_tiled() {
     return (EncodeTiledFn)p;
   }();
   return fn;
-}
-
-int env_int(const char* name, int dflt) {
-  const char* e = std::getenv(name);
-  return e ? atoi(e) : dflt;
 }
 
 template <typename T> struct FusedOps {
@@ -103,28 +88,23 @@ template <class Cfg> struct FusedImpl {
 };
 
 template <typename T> const FusedOps<T>* fused_lookup(size_t n);
-// FOURIER_B200_CFG=1 selects the other load strategy (experiments; profiles/r02_persistent_kernel_variants.txt).
 template <> const FusedOps<float>* fused_lookup<float>(size_t n) {
   if (n == ((size_t)1 << 20)) {
     // default: two 256-thread groups, TMA staging, one shared exchange buffer taken under a lock
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<float, 32, 8, 2, 8, 2, true>>::ops(8, 4);
     return FusedImpl<fused::FusedCfg<float, 32, 8, 2, 8, 1>>::ops(8, 4);
   }
   if (n == ((size_t)1 << 16)) {
     // 256 x 256 with 16 x 16 register tiles, four 128-thread groups, 64-byte tile rows as at 2^20.  Measured on B200
     // (profiles/r02_sizes_cta_and_2pow16.txt): TMA staging 56.5 %, direct loads 51.7 % (ring 128; 47 % at ring 64),
     // two launches per chunk 33.9 % of the measured HBM peak.
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<float, 16, 8, 4, 8, 4, true>>::ops(128, 64);
     return FusedImpl<fused::FusedCfg<float, 16, 8, 4, 8, 4>>::ops(128, 64);
   }
   if (n == ((size_t)1 << 18)) {
     // 512 x 512 with 32 x 16 register tiles: three 128-thread groups with TMA staging, or four with direct loads
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<float, 32, 8, 4, 8, 4, true, 16>>::ops(32, 16);
     return FusedImpl<fused::FusedCfg<float, 32, 8, 3, 8, 3, false, 16>>::ops(32, 16);
   }
   if (n == ((size_t)1 << 14)) {
     // 128 x 128 with 16 x 8 register tiles: eight 64-thread groups
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<float, 16, 8, 8, 8, 8, true, 8>>::ops(512, 256);
     return FusedImpl<fused::FusedCfg<float, 16, 8, 8, 8, 8, false, 8>>::ops(512, 256);
   }
   // Odd powers of two: N1 x 2 N1 with a different register tile per pass, same threads per FFT in both
@@ -133,19 +113,13 @@ template <> const FusedOps<float>* fused_lookup<float>(size_t n) {
     return FusedImpl<fused::FusedCfg<float, 32, 8, 2, 0, 1, false, 16, 32, 32, 32, 32, 16, true>>::ops(32, 16);   // 39 % (ring 16: 35 %, tile kernels 29 %)
   }
   if (n == ((size_t)1 << 17)) {   // 256 (16 x 16, 16 per thread) x 512 (32 x 16, 32 per thread): three 128-thread groups
-    if (env_int("FOURIER_B200_CFG", 0) == 1)
-      return FusedImpl<fused::FusedCfg<float, 16, 8, 4, 8, 4, true, 16, 32, 16, 16, 32>>::ops(64, 32);
     return FusedImpl<fused::FusedCfg<float, 16, 8, 3, 8, 3, false, 16, 32, 16, 16, 32>>::ops(64, 32);
   }
   if (n == ((size_t)1 << 15)) {   // 128 (16 x 8, 16 per thread) x 256 (16 x 16, 32 per thread): six 64-thread groups
-    if (env_int("FOURIER_B200_CFG", 0) == 1)
-      return FusedImpl<fused::FusedCfg<float, 16, 8, 8, 8, 8, true, 8, 16, 16, 16, 32>>::ops(256, 128);
     return FusedImpl<fused::FusedCfg<float, 16, 8, 6, 8, 6, false, 8, 16, 16, 16, 32>>::ops(256, 128);
   }
   // (f32 2^12 = 64 x 64 was tried on the persistent kernel: 39.0 % against 41.7 % for the two-launch tile kernels)
   if (n == ((size_t)1 << 13)) {   // 64 (8 x 8, 8 per thread) x 128 (16 x 8, 16 per thread): eight 64-thread groups
-    if (env_int("FOURIER_B200_CFG", 0) == 1)
-      return FusedImpl<fused::FusedCfg<float, 8, 8, 8, 8, 8, true, 8, 16, 8, 8, 16>>::ops(512, 256);
     return FusedImpl<fused::FusedCfg<float, 8, 8, 8, 8, 8, false, 8, 16, 8, 8, 16>>::ops(512, 256);
   }
   return nullptr;
@@ -156,22 +130,17 @@ template <> const FusedOps<double>* fused_lookup<double>(size_t n) {
     // (62.5 % / 59.9 % at batch 2048, 57.9 % / 58.8 % at 16384); at the BASELINE batch of 65536, where the run is
     // power-capped at ~1760 MHz, staging wins twice out of two A/B pairs: 56.5 / 57.4 % against 54.3 / 54.4 %
     // (profiles/r02_c3_staged_vs_direct.txt).
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<double, 16, 8, 4, 4, 4, true>>::ops(64, 32);
     return FusedImpl<fused::FusedCfg<double, 16, 8, 3, 4, 3>>::ops(64, 32);
   }
   if (n == ((size_t)1 << 14)) {
     // 128 x 128 with 16 x 8 register tiles: four 64-thread groups with TMA staging, or eight loading directly
     // measured: four groups with TMA staging 62.0 %, eight groups loading directly 53.7 %, tile kernels 37.7 %
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<double, 16, 8, 8, 4, 8, true, 8>>::ops(256, 128);
     return FusedImpl<fused::FusedCfg<double, 16, 8, 4, 4, 4, false, 8>>::ops(256, 128);
   }
   if (n == ((size_t)1 << 12)) {   // 64 x 64 with 8 x 8 register tiles
-    if (env_int("FOURIER_B200_CFG", 0) == 1) return FusedImpl<fused::FusedCfg<double, 8, 8, 8, 4, 8, false>>::ops(1024, 512);
     return FusedImpl<fused::FusedCfg<double, 8, 8, 8, 4, 8, true>>::ops(1024, 512);
   }
   if (n == ((size_t)1 << 13)) {   // 64 (8 x 8) x 128 (16 x 8): eight 64-thread groups loading directly
-    if (env_int("FOURIER_B200_CFG", 0) == 1)
-      return FusedImpl<fused::FusedCfg<double, 8, 8, 6, 4, 6, false, 8, 16, 8, 8, 16>>::ops(512, 256);
     return FusedImpl<fused::FusedCfg<double, 8, 8, 8, 4, 8, true, 8, 16, 8, 8, 16>>::ops(512, 256);
   }
   return nullptr;
@@ -186,8 +155,8 @@ cudaError_t Plan<T>::init_twopass() {
   FB_CHECK(ops->prepare());
   n1_ = ops->n1;
   n2_ = ops->n2;
-  FB_CHECK((upload_vec<T, TwPair<T>>(tw_a_, make_twa<T>(ops->ra1, ops->rb1))));
-  FB_CHECK((upload_vec<T, TwPair<T>>(tw_b_, make_twa<T>(ops->ra2, ops->rb2))));
+  FB_CHECK(upload(tw_a_, make_twa<T>(ops->ra1, ops->rb1)));
+  FB_CHECK(upload(tw_b_, make_twa<T>(ops->ra2, ops->rb2)));
   // inter-pass twiddles in the layout of the intermediate: T[k1*N2 + n2] = w_N^{n2*k1}
   std::vector<cpx<T>> tw2(n_);
   for (size_t k1 = 0; k1 < n1_; ++k1)
@@ -196,34 +165,28 @@ cudaError_t Plan<T>::init_twopass() {
       host_twiddle(k1 * c, n_, &re, &im);
       tw2[k1 * n2_ + c] = mk<T>((T)re, (T)im);
     }
-  FB_CHECK((upload_vec<T, cpx<T>>(tw2_, tw2)));
+  FB_CHECK(upload(tw2_, tw2));
   // transforms per chunk: the intermediate of one chunk should sit comfortably inside the L2
-  size_t mb = 32;
-  if (const char* env = std::getenv("FOURIER_B200_CHUNK_MB")) mb = (size_t)std::max(1, atoi(env));
-  chunk_ = std::max<size_t>(1, (mb << 20) / (n_ * sizeof(C)));
+  chunk_ = std::max<size_t>(1, (tuning_.chunk_mb << 20) / (n_ * sizeof(C)));
   fast_ops_ = ops;
   // the persistent fused kernel (one launch for the whole batch) where a configuration exists
   fused_ops_ = nullptr;
-  if (env_int("FOURIER_B200_FUSED", 1) != 0) {
+  if (tuning_.fused) {
     const FusedOps<T>* f = fused_lookup<T>(n_);
     if (f && f->prepare() == cudaSuccess) {
       // the persistent kernel has its own split and register tile (the tile kernels above stay as its fallback)
-      FB_CHECK((upload_vec<T, TwPair<T>>(tw_f_, make_twa<T>(f->ra, f->rb))));
-      FB_CHECK((upload_vec<T, TwPair<T>>(tw_f2_, make_twa<T>(f->ra2, f->rb2))));
+      FB_CHECK(upload(tw_f_, make_twa<T>(f->ra, f->rb)));
+      FB_CHECK(upload(tw_f2_, make_twa<T>(f->ra2, f->rb2)));
       // factored inter-pass twiddles, contiguous per pass-1 tile of `tile_c` columns:
       //   tbase[tile][col][p] = w_N^{n2*p},  tstep[tile][r][col] = w_N^{R*n2*r},  n2 = tile*tile_c + col
       std::vector<cpx<T>> tb, ts;
       make_factored_twiddles<T>(n_, f->n2, f->ra, f->rb, f->tile_c, tb, ts, f->base_pcol);
-      FB_CHECK((upload_vec<T, cpx<T>>(tbase_, tb)));
-      FB_CHECK((upload_vec<T, cpx<T>>(tstep_, ts)));
+      FB_CHECK(upload(tbase_, tb));
+      FB_CHECK(upload(tstep_, ts));
       fused_ops_ = f;
-      ring_ = std::max(2, env_int("FOURIER_B200_RING", f->default_ring));
+      ring_ = std::max(2, tuning_.ring.value_or(f->default_ring));
       while (ring_ & (ring_ - 1)) ++ring_;   // the kernel wants a power of two
-      lag_ = std::min(ring_ - 1, std::max(1, env_int("FOURIER_B200_LAG", f->default_lag)));
-      int dev = 0, sms = 148;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      sm_count_ = sms;
+      lag_ = std::min(ring_ - 1, std::max(1, tuning_.lag.value_or(f->default_lag)));
     }
   }
   return cudaSuccess;
@@ -234,9 +197,7 @@ cudaError_t Plan<T>::exec_twopass(const C* in, C* out, size_t batch, int code, c
   const auto* ops = static_cast<const TwoPassOps<T>*>(fast_ops_);
   const bool fwd = transform_is_forward(code);
   const bool do_scale = !(code == kFft || code == kUnscaledIfft);
-  T scale = (T)1;
-  if (code == kIfft) scale = (T)1 / (T)n_;
-  else if (do_scale) scale = (T)1 / std::sqrt((T)n_);
+  const T scale = scale_for<T>(code, n_);
   if (fused_ops_ && batch <= (size_t)1 << 24) {
     const auto* f = static_cast<const FusedOps<T>*>(fused_ops_);
     int ring = ring_;
@@ -253,7 +214,7 @@ cudaError_t Plan<T>::exec_twopass(const C* in, C* out, size_t batch, int code, c
     a.tbase = (const C*)tbase_.data(); a.tstep = (const C*)tstep_.data();
     a.counters = (unsigned*)counters_.data();
     a.trace = nullptr;
-    if (std::getenv("FOURIER_B200_TRACE")) {
+    if (!tuning_.trace.empty()) {
       const size_t tbytes = sizeof(long long) * 64 * fused::kTraceTiles * fused::kTracePhases;
       FB_CHECK(trace_.reserve(tbytes));
       FB_CHECK(cudaMemsetAsync(trace_.data(), 0, tbytes, s));
@@ -268,7 +229,7 @@ cudaError_t Plan<T>::exec_twopass(const C* in, C* out, size_t batch, int code, c
       std::vector<long long> h(64 * fused::kTraceTiles * fused::kTracePhases);
       FB_CHECK(cudaStreamSynchronize(s));
       FB_CHECK(cudaMemcpy(h.data(), trace_.data(), h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-      if (FILE* fp = fopen(std::getenv("FOURIER_B200_TRACE"), "w")) {
+      if (FILE* fp = fopen(tuning_.trace.c_str(), "w")) {
         for (int w = 0; w < 40; ++w)
           for (int k = 0; k < fused::kTraceTiles; ++k) {
             const long long* r = &h[((size_t)w * fused::kTraceTiles + k) * fused::kTracePhases];

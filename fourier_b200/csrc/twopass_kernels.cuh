@@ -2,7 +2,6 @@
 // path.  Shared by twopass.cu (the product) and tools/emulate.cu (CPU emulation of the same code).
 #pragma once
 
-#include <cstdlib>
 #include <vector>
 
 #include "plan.h"
@@ -145,12 +144,7 @@ using TwoPass = TwoPassG<T, Shape<R1, R1, R1, C1, PAD1>, Shape<R2, R2, R2, C2, 1
 // list of sizes behind lookup() here and behind the distributed variant of pass 2 (dist_fft.cu).
 template <class F> bool visit_config_f32(size_t n, F&& f) {
   switch (n) {
-    case (size_t)1 << 20: {
-      const char* env = std::getenv("FOURIER_B200_TILE");  // experiment knob: columns per tile
-      if (env && atoi(env) == 16) f(TwoPass<float, 32, 32, 16, 16, 0, 1, 1>{});
-      else f(TwoPass<float, 32, 32, 8, 8, 8, 2, 2>{});
-      return true;
-    }
+    case (size_t)1 << 20: f(TwoPass<float, 32, 32, 8, 8, 8, 2, 2>{}); return true;
     case (size_t)1 << 11: f(TwoPassG<float, Shape<4, 8, 8, 32, 0>, Shape<8, 8, 8, 32, 2>, 4, 4>{}); return true;
     case (size_t)1 << 12: f(TwoPassG<float, Shape<8, 8, 8, 32, 0>, Shape<8, 8, 8, 32, 2>, 4, 4>{}); return true;
     case (size_t)1 << 13: f(TwoPassG<float, Shape<8, 8, 8, 32, 0>, Shape<8, 16, 16, 16, 2>, 4, 4>{}); return true;
@@ -185,14 +179,6 @@ template <typename T> const TwoPassOps<T>* lookup(size_t n) {
   visit_config<T>(n, [&](auto g) { o = decltype(g)::ops(); });
   return o;
 }
-
-template <typename T, typename U>
-cudaError_t upload_vec(DeviceBuffer& buf, const std::vector<U>& host) {
-  cudaError_t e = buf.reserve(host.size() * sizeof(U));
-  if (e != cudaSuccess) return e;
-  return cudaMemcpy(buf.data(), host.data(), host.size() * sizeof(U), cudaMemcpyHostToDevice);
-}
-
 
 }  // namespace twopass
 }  // namespace fb200

@@ -340,21 +340,6 @@ def test_fused_paths_agree_with_general_path(real, n):
         assert rel_err(gpu_transform(fast, x, code), gpu_transform(gen, x, code)) < TOL[real]
 
 
-@pytest.mark.parametrize("real,n", [("f32", 1 << 20), ("f64", 1 << 16)])
-def test_alternative_persistent_kernel_configuration(monkeypatch, real, n):
-    # FOURIER_B200_CFG=1 (read when the plan is created) selects the other load strategy of the persistent two-pass
-    # kernel: direct global loads instead of TMA staging
-    monkeypatch.setenv("FOURIER_B200_CFG", "1")
-    x = O.fill_input(40, n, NP[real], first_transform=2)
-    alt = create(real, n)
-    monkeypatch.delenv("FOURIER_B200_CFG")
-    ref = create(real, n)
-    for code in (T.Fft, T.Ifft):
-        got = gpu_transform(alt, x, code)
-        assert rel_err(got, gpu_transform(ref, x, code)) < TOL[real]
-        assert rel_err(got[7], O.transform(x[7], int(code))) < TOL[real]
-
-
 def test_misaligned_device_pointer_is_refused():
     """ADVICE r1: the kernels use 16-byte vector accesses / TMA on device buffers; a slice that starts at an odd f32
     sample is only 8-byte aligned and must be refused up front (no launch, no sticky CUDA error)."""

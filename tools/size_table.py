@@ -1,7 +1,7 @@
 """Throughput table over transform sizes (one B200): path, kernel, samples/s, fraction of the measured HBM peak, launches
 per transform call, rel. error of one transform vs the oracle.
     PYTHONPATH=. python tools/size_table.py f32 243 729 2187 65536 ...     (sizes; 2^k may be written as 2^k)
-Environment knobs of the library (FOURIER_B200_CFG, _FUSED, _TWOPASS, _RING, _LAG) apply and are echoed."""
+Environment knobs of the library (FOURIER_B200_FUSED, _TWOPASS, _RING, _LAG) apply and are echoed."""
 import json
 import os
 import sys
